@@ -5,6 +5,10 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1     # CPU oracle arm
+    python bench.py --gpus 1 --steps 20 --warmup 5 --dump-outputs DIR  # also write the last timed step's outputs
+
+Every timed loop of train steps (the main region, the per-step distribution, the end-to-end loop, the per-kernel
+timing and the `strong` / `tt_sh25` extras) runs --steps steps.
 
 Workload (config.workload): BASELINE.json configs[1] — nerf_sh/config/blender (SH16, 64 coarse + 128
 fine samples = 256 MLP evaluations per ray, white background, sparsity loss on 10,000 points), synthetic
@@ -159,6 +163,21 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, model, state, world):
+    """Write what the last timed train_step left its caller, as float32 / float64 .npy files: the updated parameters
+    (params), the Adam moments (adam_m, adam_v), the step's rank-averaged gradient (grads) and its Stats
+    (stats: loss, psnr, loss_c, loss_sp, psnr_c, weight_l2).  About 16 MB for SH16."""
+    from plenoctree_b200.nerf import train as T
+    torch.cuda.synchronize()
+    st = T.stats_from_raw(state.stats_raw / world, RAYS, 1e-3, NSP, True)
+    st = st._replace(weight_l2=float((model.params.double() ** 2).sum() / model.params.numel()))
+    arrays = {"params": model.params, "adam_m": state.m, "adam_v": state.v, "grads": state.grads / world}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "stats.npy"), np.array(st, dtype=np.float64))
+
+
 def cpu_baseline_sample():
     from oracle import nerf_sh_oracle as O
     from plenoctree_b200.nerf.rays import random_rays_np   # numpy only: the CPU arm maps no repo .so
@@ -199,7 +218,15 @@ def main():
     ap.add_argument("--workload", default="blender", choices=["blender", "tt"],
                     help="blender = BASELINE configs[1] (SH16, near/far 2/6; the default and the quoted metric); "
                          "tt = configs[2] (SH25, near/far 0/4, sparsity radius 5 / length 0.2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the parameters, Adam moments, gradient and loss statistics of "
+                         "the last timed step as DIR/<name>.npy (inputs are seeded: the same arguments give the same "
+                         "inputs, so two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -313,9 +340,11 @@ def main():
     launches0 = _lib.lib.pob_launch_count()
     ms_total = timed(step_resident, W)
     launches = int(_lib.lib.pob_launch_count() - launches0)
-    # ---- per-step distribution over a longer run (the contract region above is K steps long; the driver's K = 20
-    # is 80 ms): every step bracketed by its own pair of events, no host sync inside the loop
-    ND = 100
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, state, world)
+    # ---- per-step distribution over K further steps: every step bracketed by its own pair of events, no host sync
+    # inside the loop
+    ND = K
     evs = [torch.cuda.Event(enable_timing=True) for _ in range(ND + 1)]
     barrier()
     evs[0].record()
@@ -335,9 +364,9 @@ def main():
     assert len(losses) - n_before == K and all(np.isfinite(losses[n_before:])), "e2e loop must read every step's loss"
     if sampler:
         sampler.stop()
-    # ---- per-kernel-class timing (CUDA events around every launch), separate short run ----
+    # ---- per-kernel-class timing (CUDA events around every launch), a separate run of K steps ----
     _lib.lib.pob_timing_enable(1)
-    nprof = min(K, 10)
+    nprof = K
     for i in range(nprof):
         step_resident(W + i)
     ms_ph = (ctypes.c_double * 5)()
@@ -373,8 +402,8 @@ def main():
     extras = {}
     if not args.no_extras:
         import bench_extras as X
-        for key, fn in (("strong", lambda: X.strong_scaling(dev, peaks["tflops"], steps=max(K, 20))),
-                        ("tt_sh25", lambda: X.strong_scaling(dev, peaks["tflops"], steps=max(K, 20), tt=True)),
+        for key, fn in (("strong", lambda: X.strong_scaling(dev, peaks["tflops"], steps=K)),
+                        ("tt_sh25", lambda: X.strong_scaling(dev, peaks["tflops"], steps=K, tt=True)),
                         ("c4_extraction", lambda: X.c4_extraction(dev, peaks["tflops"])),
                         ("c5_octree_opt", lambda: X.c5_octree_opt(dev)),
                         ("render_eval", lambda: X.render_eval(dev))):
