@@ -169,17 +169,13 @@ typedef struct pob_train_hparams {
 
 /* grad_flat [num_mlps * pob_param_count] (MLP_0 then MLP_1, reference flat order), per-rank gradient of
  *   mean((rgb_f-px)^2) + mean((rgb_c-px)^2) + sparsity_weight*(1-mean(exp(-len*relu(sigma(p)))))
- * stats [8] (device): [0] sum (rgb_fine-px)^2, [1] sum (rgb_coarse-px)^2, [2] sum exp(-len*relu(sigma)).
- * The backward of MLP_0 (coarse level) is finished first; mlp0_done_event (a cudaEvent_t, or NULL) is recorded on
- * `stream` once grad_flat[0 : pob_param_count) is final, so that the caller can all-reduce that bucket on another
- * stream while the MLP_1 backward (three quarters of the work) is still running (the two branches are independent:
- * stop_gradient, nerf_sh/nerf/model_utils.py:286). */
+ * stats [8] (device): [0] sum (rgb_fine-px)^2, [1] sum (rgb_coarse-px)^2, [2] sum exp(-len*relu(sigma)). */
 int pob_loss_and_grad(const pob_render_config* cfg, const pob_train_hparams* hp, const void* packed_coarse_dev,
                       const void* packed_fine_dev, const float* origins_dev, const float* directions_dev,
                       const float* viewdirs_dev, const float* pixels_dev, int n_rays, const float* z_base_dev,
                       const float* t_rand_dev, const float* u_dev, int u_per_ray, const float* z_fine_dev,
                       const float* sp_points_dev, float* grad_flat_dev, float* stats_dev, void* workspace_dev,
-                      void* mlp0_done_event, void* stream);
+                      void* stream);
 
 /* flax.optim.Adam (beta1 .9, beta2 .999, eps 1e-8; nerf_sh/nerf/models.py:44) on the flat buffers of
  * num_mlps MLPs, g = grad*grad_mult + weight_decay_coef*param, then re-packs the operand blobs.
@@ -195,16 +191,16 @@ int pob_adam_update(int sh_deg, int num_mlps, float* params_dev, const float* gr
  * save_*_dev (all or none; sized like the training workspace: 512 KB, 16 KB and 4 KB per 128 samples) turn
  * on the training-mode stores so their cost shows in the trace. */
 int pob_debug_trace_fwd(const void* packed_dev, int sh_deg, const float* points_dev, int64_t m,
-                        float* raw_sigma_dev, unsigned long long* trace_dev, int debug_flags, void* save_h_dev,
+                        float* raw_sigma_dev, unsigned long long* trace_dev, void* save_h_dev,
                         void* save_e_dev, void* save_mask_dev, void* stream);
 
 /* Profiling aid: one mlp_bwd launch (dgrad chain, FP16) on caller-provided inputs — per-sample gradients g_dev
  * [m,4], view directions [m,3], relu masks (4 KB per 128 samples and layer), dZ / dO destinations sized like the
  * training workspace — recording clock64() stamps of CTA 0 into trace_dev[2][256] (role 0 = MMA issuer, 1 = first
- * epilogue warp of tile X); scripts/trace_summary.py.  debug_flags: timing experiments (results invalid). */
+ * epilogue warp of tile X); scripts/trace_bwd.py. */
 int pob_debug_trace_bwd(const void* packed_dev, int sh_deg, int64_t m, const float* g_dev, const float* viewdirs_dev,
                         const void* mask_dev, void* save_dz_dev, void* save_do_dev, unsigned long long* trace_dev,
-                        int debug_flags, void* stream);
+                        void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * PlenOctree side (SURVEY.md §8 rows a13-middle and a15).  These entry points stand where the

@@ -27,8 +27,8 @@ SIGNATURES = {
     "pob_packed_bytes": (_i64, [_i]),
     "pob_pack_weights": (_i, [_fp, _i, _vp, _vp]),
     "pob_eval_points_raw": (_i, [_vp, _i, _fp, _i64, _fp, _fp, _i, _vp]),
-    "pob_debug_trace_fwd": (_i, [_vp, _i, _fp, _i64, _fp, _vp, _i, _vp, _vp, _vp, _vp]),
-    "pob_debug_trace_bwd": (_i, [_vp, _i, _i64, _fp, _fp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "pob_debug_trace_fwd": (_i, [_vp, _i, _fp, _i64, _fp, _vp, _vp, _vp, _vp, _vp]),
+    "pob_debug_trace_bwd": (_i, [_vp, _i, _i64, _fp, _fp, _vp, _vp, _vp, _vp, _vp]),
     "pob_eval_points": (_i, [_vp, _i, _fp, _fp, _i64, _fp, _i, _vp]),
     "pob_eval_cells_mean": (_i, [_vp, _i, _fp, _i64, _i, _fp, _i, _vp]),
     "pob_eval_grid": (_i, [_vp, _i, _i, _i, _i, _i, _i, _c.POINTER(_c.c_float), _c.POINTER(_c.c_float),
@@ -42,7 +42,7 @@ SIGNATURES = {
     "pob_workspace_bytes": (_i64, [_vp, _i]),
     "pob_render_rays": (_i, [_vp, _vp, _vp, _fp, _fp, _fp, _i, _fp, _fp, _fp, _i, _fp, _fp, _fp, _vp, _i, _vp]),
     "pob_loss_and_grad": (_i, [_vp, _vp, _vp, _vp, _fp, _fp, _fp, _fp, _i, _fp, _fp, _fp, _i, _fp, _fp, _fp, _fp,
-                               _vp, _vp, _vp]),
+                               _vp, _vp]),
     "pob_adam_update": (_i, [_i, _i, _fp, _fp, _fp, _fp, _c.c_float, _c.c_float, _fp, _c.c_float, _c.c_float,
                              _vp, _vp, _vp]),
     "pob_octree_render": (_i, [_vp, _vp, _fp, _fp, _fp, _i64, _vp, _i, _i, _fp, _vp, _vp]),

@@ -135,7 +135,9 @@ pob::FwdParams pob_base_params(const void* packed, int sh_deg) { return base_par
 
 extern "C" {
 
-int pob_abi_version(void) { return 4; }   // 4: pob_loss_and_grad(mlp0_done_event), pob_adam_update(lr_step_dev); 3: CTA-pair kernels
+// 5: pob_loss_and_grad without its MLP_0 event, pob_debug_trace_fwd / _bwd without debug flags;
+// 4: pob_loss_and_grad(MLP_0 event), pob_adam_update(lr_step_dev); 3: CTA-pair kernels
+int pob_abi_version(void) { return 5; }
 
 long long pob_launch_count(void) { return g_launches.load(); }
 
@@ -198,13 +200,12 @@ int pob_eval_points_raw(const void* packed_dev, int sh_deg, const float* points_
   pob_count_launch();
   PobPhaseTimer _t(POB_PH_FWD, (cudaStream_t)stream);
   POB_CUDA("pob_eval_points_raw",
-           pob::launch_mlp_fwd(p, precision, precision == POB_PREC_FP16X3, sm_count(),
-                               (cudaStream_t)stream));
+           pob::launch_mlp_fwd(p, precision, sm_count(), (cudaStream_t)stream));
   return 0;
 }
 
 int pob_debug_trace_fwd(const void* packed_dev, int sh_deg, const float* points_dev, int64_t m,
-                        float* raw_sigma_dev, unsigned long long* trace_dev, int debug_flags, void* save_h_dev,
+                        float* raw_sigma_dev, unsigned long long* trace_dev, void* save_h_dev,
                         void* save_e_dev, void* save_mask_dev, void* stream) {
   if (int e = check_common("pob_debug_trace_fwd", packed_dev, sh_deg, POB_PREC_FP16)) return e;
   if (!points_dev || !raw_sigma_dev || !trace_dev || m <= 0) return fail("pob_debug_trace_fwd", "bad arguments");
@@ -215,17 +216,16 @@ int pob_debug_trace_fwd(const void* packed_dev, int sh_deg, const float* points_
   p.out_mode = pob::OUT_SIGMA;
   p.out_sigma = raw_sigma_dev;
   p.trace = trace_dev;
-  p.debug_flags = debug_flags;
   p.save_h = static_cast<uint8_t*>(save_h_dev);
   p.save_e = static_cast<uint8_t*>(save_e_dev);
   p.save_mask = static_cast<uint32_t*>(save_mask_dev);
-  POB_CUDA("pob_debug_trace_fwd", pob::launch_mlp_fwd(p, 1, false, sm_count(), (cudaStream_t)stream));
+  POB_CUDA("pob_debug_trace_fwd", pob::launch_mlp_fwd(p, 1, sm_count(), (cudaStream_t)stream));
   return 0;
 }
 
 int pob_debug_trace_bwd(const void* packed_dev, int sh_deg, int64_t m, const float* g_dev, const float* viewdirs_dev,
                         const void* mask_dev, void* save_dz_dev, void* save_do_dev, unsigned long long* trace_dev,
-                        int debug_flags, void* stream) {
+                        void* stream) {
   if (int e = check_common("pob_debug_trace_bwd", packed_dev, sh_deg, POB_PREC_FP16)) return e;
   if (!g_dev || !viewdirs_dev || !mask_dev || !save_dz_dev || !save_do_dev || m <= 0)
     return fail("pob_debug_trace_bwd", "bad arguments");
@@ -245,7 +245,6 @@ int pob_debug_trace_bwd(const void* packed_dev, int sh_deg, int64_t m, const flo
   b.save_dz = static_cast<uint8_t*>(save_dz_dev);
   b.save_do = static_cast<uint8_t*>(save_do_dev);
   b.trace = trace_dev;
-  b.debug_flags = debug_flags;
   POB_CUDA("pob_debug_trace_bwd", pob::launch_mlp_bwd(b, sm_count(), (cudaStream_t)stream));
   return 0;
 }
@@ -269,8 +268,7 @@ int pob_eval_points(const void* packed_dev, int sh_deg, const float* points_dev,
   pob_count_launch();
   PobPhaseTimer _t(POB_PH_FWD, (cudaStream_t)stream);
   POB_CUDA("pob_eval_points",
-           pob::launch_mlp_fwd(p, precision, precision == POB_PREC_FP16X3, sm_count(),
-                               (cudaStream_t)stream));
+           pob::launch_mlp_fwd(p, precision, sm_count(), (cudaStream_t)stream));
   return 0;
 }
 
@@ -292,7 +290,7 @@ int pob_eval_cells_mean(const void* packed_dev, int sh_deg, const float* points_
   pob_count_launch();
   PobPhaseTimer _t(POB_PH_FWD, (cudaStream_t)stream);
   POB_CUDA("pob_eval_cells_mean",
-           pob::launch_mlp_fwd(p, precision, precision == POB_PREC_FP16X3, sm_count(), (cudaStream_t)stream));
+           pob::launch_mlp_fwd(p, precision, sm_count(), (cudaStream_t)stream));
   return 0;
 }
 
@@ -325,8 +323,7 @@ int pob_eval_grid(const void* packed_dev, int sh_deg, int reso, int x0, int nx, 
   pob_count_launch();
   PobPhaseTimer _t(POB_PH_FWD, (cudaStream_t)stream);
   POB_CUDA("pob_eval_grid",
-           pob::launch_mlp_fwd(p, precision, precision == POB_PREC_FP16X3, sm_count(),
-                               (cudaStream_t)stream));
+           pob::launch_mlp_fwd(p, precision, sm_count(), (cudaStream_t)stream));
   return 0;
 }
 

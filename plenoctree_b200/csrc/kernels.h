@@ -53,8 +53,6 @@ struct FwdParams {
   uint32_t* save_mask;         // [8][ntile*128][8] relu masks (bit i of word c = col 32c+i)
   // ---- optional cycle trace of CTA 0 (debug/profiling; null = off): [3 roles][256] clock64 stamps
   unsigned long long* trace;
-  int debug_flags;             // timing experiments only (results invalid; pob_debug_trace_fwd): 8 no weight loads,
-                               // 16 h stores to one L2-resident tile per CTA, 32 drop in-epilogue stores, 64 drop deferred stores
 };
 
 // padded heads width for K spherical-harmonic coefficients per channel
@@ -64,12 +62,9 @@ inline size_t fwd_image_bytes(int NH) { return size_t(66) * 16384 + size_t(9) * 
 // bytes of one dgrad weight image: heads (ceil(NH/32) slots) + layers 7..1 (8 slots each)
 inline size_t bwd_image_bytes(int NH) { return size_t((NH + 31) / 32 + 7 * 8) * 16384; }
 
-// precision: 1 = single fp16 pass (10-bit mantissa operands, fp32 accumulate),
-//            3 = error-compensated 3-pass split (hi*hi + lo*hi + hi*lo)
-cudaError_t launch_mlp_fwd(const FwdParams& p, int nsplit, bool precise_sin, int num_sms,
-                           cudaStream_t stream);
-// single-pass forward / dgrad kernels run as CTA pairs (cta_group::2) unless POB_PAIR=0
-bool pair_mode_enabled();
+// precision: 1 = single fp16 pass (10-bit mantissa operands, fp32 accumulate; CTA pairs, cta_group::2),
+//            3 = error-compensated 3-pass split (hi*hi + lo*hi + hi*lo; single CTAs)
+cudaError_t launch_mlp_fwd(const FwdParams& p, int nsplit, int num_sms, cudaStream_t stream);
 
 // flat fp32 parameters of one MLP in reference order (Dense_0..Dense_9: kernel [in,out] then
 // bias) -> packed images.  `nparams` = param_count(K).
@@ -121,9 +116,8 @@ struct BwdParams {
   uint8_t* save_dz;         // [ntile][8][64 KB]
   uint8_t* save_do;         // [ntile][32 KB]
   unsigned long long* trace;   // optional cycle trace of CTA 0 (null = off): [2 roles][256] clock64 stamps
-  int debug_flags;          // timing experiments only (results invalid): 1 no tile copy-out, 2 no mask loads
 };
-cudaError_t launch_mlp_bwd(const BwdParams& p, int num_sms, cudaStream_t stream);
+cudaError_t launch_mlp_bwd(const BwdParams& p, int num_sms, cudaStream_t stream);   // CTA pairs
 
 // ---- mlp_wgrad.cu ---------------------------------------------------------------------------
 constexpr int WG_PARTIAL_FLOATS = 65536 + 256;

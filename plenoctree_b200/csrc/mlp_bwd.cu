@@ -17,11 +17,9 @@
 // copy warps; those pull it into registers half a tile at a time (the shared-memory tile is free again ~2.6 k
 // cycles after the hand-over, well before the next epilogue needs it) and let the stores drain from registers.
 //
-// PAIR (default): two CTAs of a cluster share one tcgen05.mma.cta_group::2 stream over four tiles
-// (512 samples per iteration), each CTA holding half of every transposed-weight slot — same protocol
-// as mlp_fwd.cu (leader issues, peer relays landed half-slots, commits multicast to both CTAs).
-#include <cstdlib>
-
+// Two CTAs of a cluster share one tcgen05.mma.cta_group::2 stream over four tiles (512 samples per
+// iteration), each CTA holding half of every transposed-weight slot — same protocol as mlp_fwd.cu
+// (leader issues, peer relays landed half-slots, commits multicast to both CTAs).
 #include "common.cuh"
 #include "kernels.h"
 
@@ -33,8 +31,8 @@ constexpr int BWD_THREADS = 576;
 constexpr int BWD_COPY_WARP0 = 10;     // first copy-out warp
 constexpr int BWD_PRODUCER_WARP = 8;
 constexpr int BWD_MMA_WARP = 9;
-constexpr int BWD_WSLOTS = 6;            // 16 KB slots (single CTA) or twice as many 8 KB half-slots (pair)
-constexpr int BWD_MAX_RING = 2 * BWD_WSLOTS;
+constexpr int BWD_WSLOTS = 6;            // 16 KB of shared memory each, streamed as two 8 KB half-slots
+constexpr int BWD_RING = 2 * BWD_WSLOTS; // ring of 8 KB half-slots: this CTA's half of each weight slot
 
 constexpr uint32_t SB_A0 = 0;
 constexpr uint32_t SB_A1 = SB_A0 + A_TILE_BYTES;
@@ -42,8 +40,8 @@ constexpr uint32_t SB_W = SB_A1 + A_TILE_BYTES;
 constexpr uint32_t SB_TOTAL = SB_W + BWD_WSLOTS * WSLOT_BYTES;  // 128K + 96K = 224K
 
 struct BwdBarriers {
-  uint64_t full[BWD_MAX_RING];
-  uint64_t empty[BWD_MAX_RING];
+  uint64_t full[BWD_RING];
+  uint64_t empty[BWD_RING];
   uint64_t a_ready[2];
   uint64_t d_ready[2];
   uint64_t c_ready[2];   // epilogue group -> copy warps: tile written (4 arrivals)
@@ -56,33 +54,32 @@ __device__ __forceinline__ void bwd_stamp(unsigned long long* tr, int role, uint
 
 }  // namespace
 
-template <bool PAIR>
 __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
   __shared__ __align__(8) BwdBarriers bars;
   __shared__ uint32_t tmem_base_s;
 
-  constexpr int TILES_PER_ITER = PAIR ? 4 : 2;
-  constexpr int RING = PAIR ? BWD_MAX_RING : BWD_WSLOTS;
-  constexpr uint32_t RSLOT_BYTES = PAIR ? WSLOT_BYTES / 2 : WSLOT_BYTES;
+  constexpr int TILES_PER_ITER = 4;
+  constexpr int RING = BWD_RING;
+  constexpr uint32_t RSLOT_BYTES = WSLOT_BYTES / 2;
   const long long mrows = padded_rows(p.M);                       // rows of the mask / tile arrays (4-tile units)
   const long long num_iters = mrows / (TILES_PER_ITER * TILE_M);  // padded tiles get zero gradients, not garbage
   const uint32_t warp = warp_id(), lane = lane_id();
   const uint32_t sbase = smem_u32(smem);
-  const uint32_t rank = PAIR ? cluster_ctarank() : 0u;
-  const long long unit = PAIR ? (long long)(blockIdx.x >> 1) : (long long)blockIdx.x;
-  const long long nunits = PAIR ? (long long)(gridDim.x >> 1) : (long long)gridDim.x;
+  const uint32_t rank = cluster_ctarank();                        // 0 = leader (issues the MMAs)
+  const long long unit = (long long)(blockIdx.x >> 1);
+  const long long nunits = (long long)(gridDim.x >> 1);
   const int NH = p.NH;
   const int hs = (NH + 31) / 32;            // K slots of the heads dgrad
   const int do_chunks = (NH + 63) / 64;     // 64-wide chunks of the dO tile image
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < RING; ++i) {
-      // pair mode, leader: a slot is full when its own half has landed AND the peer has reported its half
-      mbar_init(smem_u32(&bars.full[i]), (PAIR && rank == 0) ? 2 : 1);
+      // leader: a slot is full when its own half has landed AND the peer has reported its half
+      mbar_init(smem_u32(&bars.full[i]), rank == 0 ? 2 : 1);
       mbar_init(smem_u32(&bars.empty[i]), 1);
     }
     for (int g = 0; g < 2; ++g) {
-      mbar_init(smem_u32(&bars.a_ready[g]), PAIR ? 8 : 4);
+      mbar_init(smem_u32(&bars.a_ready[g]), 8);   // 4 own epilogue warps + the peer's 4 (remote)
       mbar_init(smem_u32(&bars.d_ready[g]), 1);
       mbar_init(smem_u32(&bars.c_ready[g]), 4);
       mbar_init(smem_u32(&bars.c_free[g][0]), 4);
@@ -90,11 +87,8 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
     }
     fence_mbar_init();
   }
-  if (PAIR) cluster_sync_all();
-  if (warp == BWD_PRODUCER_WARP) {
-    if (PAIR) tmem_alloc_pair(smem_u32(&tmem_base_s), 512);
-    else tmem_alloc(smem_u32(&tmem_base_s), 512);
-  }
+  cluster_sync_all();   // both CTAs' barriers exist before any remote arrive / multicast commit
+  if (warp == BWD_PRODUCER_WARP) tmem_alloc_pair(smem_u32(&tmem_base_s), 512);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -104,7 +98,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
   };
 
   if (warp == BWD_PRODUCER_WARP) {
-    // whole-warp control flow, one elected lane issues (see mlp_fwd.cu); pair: this CTA's half of every slot
+    // whole-warp control flow, one elected lane issues (see mlp_fwd.cu); this CTA's half of every slot
     uint32_t slot = 0, phase = 0;
     const int nslots = hs + 7 * 8;
     for (long long it = unit; it < num_iters; it += nunits) {
@@ -124,7 +118,8 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
     }
   } else if (warp == BWD_MMA_WARP) {
     uint32_t slot = 0, phase = 0, aphase = 0;
-    if (PAIR && rank != 0) {
+    if (rank != 0) {
+      // peer CTA: no MMAs to issue; relay every landed half-slot to the leader's full barrier
       const uint32_t pfull0 = mapa_cluster(smem_u32(&bars.full[0]), 0);
       const int nslots = hs + 7 * 8;
       for (long long it = unit; it < num_iters; it += nunits) {
@@ -143,8 +138,8 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
       // epilogue drains X's accumulator and writes X's next operand tile, and vice versa, so the tensor pipe
       // does not idle through the epilogues (lock-step tiles: MMA 4.4 k + epilogue 1.8 k cycles per GEMM pair).
       // Every weight slot is streamed once and read twice, by X and — one GEMM (ns slots) later — by Y; the
-      // ring (12 half-slots in pair mode) holds the GEMM's 8 slots plus 4 of prefetch.
-      const uint32_t idesc = make_idesc_f16(PAIR ? 2 * TILE_M : TILE_M, WIDTH);
+      // ring of 12 half-slots holds the GEMM's 8 slots plus 4 of prefetch.
+      const uint32_t idesc = make_idesc_f16(2 * TILE_M, WIDTH);
       constexpr uint64_t A_HI = make_sdesc_hi(1024, LAYOUT_SW128) | (uint64_t(1) << 16);
       constexpr uint64_t W_HI = make_sdesc_hi(512, LAYOUT_SW64) | (uint64_t(1) << 16);
       uint32_t tn = 0;
@@ -152,8 +147,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
       for (long long it = unit; it < num_iters; it += nunits) {
         for (int grp = 0; grp < 8; ++grp) {      // heads, then Dense_7 .. Dense_1
           const int ns = (grp == 0) ? hs : 8;
-          // slots per turn: the whole GEMM when the ring can hold it (pair mode: 12 half-slots), else 2
-          constexpr int TURN = PAIR ? 8 : 2;
+          constexpr int TURN = 8;   // slots per turn: the whole GEMM (the ring holds it)
           for (int j0 = 0; j0 < ns; j0 += TURN) {
             const int j1 = j0 + TURN < ns ? j0 + TURN : ns;
 #pragma unroll
@@ -174,17 +168,10 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
                   const uint32_t a_base = sbase + (g ? SB_A1 : SB_A0) + a_off;
                   const uint64_t ad0 = A_HI | uint64_t((a_base >> 4) & 0x3FFF);
                   const uint32_t d = tmem + uint32_t(g) * 256u;
-                  if (PAIR) {
-                    umma_f16_pair(d, ad0, bd0, idesc, j != 0);
-                    umma_f16_pair(d, ad0 + 2, bd0 + 2, idesc, 1u);
-                    if (j == ns - 1) umma_commit_pair(smem_u32(&bars.d_ready[g]), 0x3);
-                    if (g == 1) umma_commit_pair(smem_u32(&bars.empty[rs]), 0x3);
-                  } else {
-                    umma_f16(d, ad0, bd0, idesc, j != 0);
-                    umma_f16(d, ad0 + 2, bd0 + 2, idesc, 1u);
-                    if (j == ns - 1) umma_commit(smem_u32(&bars.d_ready[g]));
-                    if (g == 1) umma_commit(smem_u32(&bars.empty[rs]));
-                  }
+                  umma_f16_pair(d, ad0, bd0, idesc, j != 0);
+                  umma_f16_pair(d, ad0 + 2, bd0 + 2, idesc, 1u);
+                  if (j == ns - 1) umma_commit_pair(smem_u32(&bars.d_ready[g]), 0x3);
+                  if (g == 1) umma_commit_pair(smem_u32(&bars.empty[rs]), 0x3);
                 }
                 __syncwarp();
                 if (++rs == RING) {
@@ -212,7 +199,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
     const uint8_t* const a_tile = smem + (g ? SB_A1 : SB_A0);
     uint32_t cphase = 0;
     for (long long it = unit; it < num_iters; it += nunits) {
-      const long long tile_idx = it * TILES_PER_ITER + (PAIR ? int(rank) * 2 : 0) + g;
+      const long long tile_idx = it * TILES_PER_ITER + int(rank) * 2 + g;
       for (int k = 0; k <= NUM_TRUNK; ++k) {          // dO, dZ_7 .. dZ_0
         const uint32_t half = (k == 0 ? uint32_t(do_chunks) * A_CHUNK_BYTES : uint32_t(A_TILE_BYTES)) / 2;   // 8, 16 or 32 KB
         const uint32_t share = half / 4;                                                                     // 2, 4 or 8 KB
@@ -231,11 +218,9 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
             if (i < nu) r[i] = *reinterpret_cast<const uint4*>(src + b * half + i * 512);
           __syncwarp();
           if (lane == 0) mbar_arrive(smem_u32(&bars.c_free[g][b]));
-          if (!(p.debug_flags & 1)) {
 #pragma unroll
-            for (int i = 0; i < 16; ++i)
-              if (i < nu) *reinterpret_cast<uint4*>(dst + b * half + i * 512) = r[i];
-          }
+          for (int i = 0; i < 16; ++i)
+            if (i < nu) *reinterpret_cast<uint4*>(dst + b * half + i * 512) = r[i];
         }
       }
     }
@@ -249,7 +234,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
     const uint32_t d_tmem = tmem + (uint32_t((warp & 3) * 32) << 16) + uint32_t(g) * 256u;
     uint32_t dphase = 0, fphase = 0;
     bool first_tile = true;
-    const uint32_t a_ready_addr = (PAIR && rank != 0) ? mapa_cluster(smem_u32(&bars.a_ready[g]), 0)
+    const uint32_t a_ready_addr = rank != 0 ? mapa_cluster(smem_u32(&bars.a_ready[g]), 0)
                                                       : smem_u32(&bars.a_ready[g]);
     // hand the finished tile to the MMA warp (unless it is dZ_0: no GEMM follows) and to the copy warps
     auto hand_over = [&](bool to_mma) {
@@ -257,10 +242,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
       tc_fence_before();
       __syncwarp();
       if (lane == 0) {
-        if (to_mma) {
-          if (PAIR) mbar_arrive_cluster_any(a_ready_addr, rank != 0);
-          else mbar_arrive(a_ready_addr);
-        }
+        if (to_mma) mbar_arrive_cluster_any(a_ready_addr, rank != 0);
         mbar_arrive(smem_u32(&bars.c_ready[g]));
       }
     };
@@ -276,7 +258,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
 
     // Global loads of an iteration (per-sample gradient, view direction, ReLU masks) are issued one step ahead
     // of their use.
-    auto sample_of = [&](long long it_) { return (it_ * TILES_PER_ITER + (PAIR ? int(rank) * 2 : 0) + g) * TILE_M + row; };
+    auto sample_of = [&](long long it_) { return (it_ * TILES_PER_ITER + int(rank) * 2 + g) * TILE_M + row; };
     auto mask_ptr = [&](int l, long long s_) { return reinterpret_cast<const uint4*>(p.mask + (size_t(l) * mrows + s_) * 8); };
     float4 gq_n = make_float4(0.f, 0.f, 0.f, 0.f);
     float vd_n[3] = {0.f, 0.f, 1.f};
@@ -296,7 +278,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
     if (unit < num_iters) prefetch_iter(unit);
 
     for (long long it = unit; it < num_iters; it += nunits) {
-      const long long tile_idx = it * TILES_PER_ITER + (PAIR ? int(rank) * 2 : 0) + g;
+      const long long tile_idx = it * TILES_PER_ITER + int(rank) * 2 + g;
       const long long s = tile_idx * TILE_M + row;
       // ---- dO row from the per-sample gradient and the SH basis ----
       {
@@ -344,8 +326,7 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
         dphase ^= 1;
         tc_fence_after();
         bwd_stamp(tre, 1, tn);                          // d_ready observed
-        if (p.debug_flags & 2) {
-        } else if (l > 0) {
+        if (l > 0) {
           mn0 = __ldg(mask_ptr(l - 1, s));
           mn1 = __ldg(mask_ptr(l - 1, s) + 1);
         } else if (it + nunits < num_iters) {
@@ -390,42 +371,25 @@ __device__ __forceinline__ void bwd_body(const BwdParams& p, uint8_t* smem) {
   }
 
   tc_fence_before();
-  if (PAIR) {
-    cluster_sync_all();
-    if (warp == BWD_PRODUCER_WARP) tmem_dealloc_pair(tmem, 512);
-  } else {
-    __syncthreads();
-    if (warp == BWD_PRODUCER_WARP) tmem_dealloc(tmem, 512);
-  }
-}
-
-__global__ void __launch_bounds__(BWD_THREADS, 1) mlp_bwd_kernel(const __grid_constant__ BwdParams p) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  bwd_body<false>(p, smem);
+  // every epilogue warp has seen the last d_ready = every MMA that reads either CTA's shared memory is done
+  cluster_sync_all();
+  if (warp == BWD_PRODUCER_WARP) tmem_dealloc_pair(tmem, 512);
 }
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(BWD_THREADS, 1)
 mlp_bwd_pair_kernel(const __grid_constant__ BwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
-  bwd_body<true>(p, smem);
+  bwd_body(p, smem);
 }
 
 cudaError_t launch_mlp_bwd(const BwdParams& p, int num_sms, cudaStream_t stream) {
   if (p.M <= 0) return cudaSuccess;
-  const bool pair = num_sms >= 2 && pair_mode_enabled();
-  const long long iters = padded_rows(p.M) / ((pair ? 4 : 2) * TILE_M);
-  const int units = pair ? num_sms / 2 : num_sms;
-  const int grid = int(iters < units ? iters : units) * (pair ? 2 : 1);
-  cudaError_t e;
-  if (pair) {
-    e = cudaFuncSetAttribute(mlp_bwd_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SB_TOTAL);
-    if (e != cudaSuccess) return e;
-    mlp_bwd_pair_kernel<<<grid, BWD_THREADS, SB_TOTAL, stream>>>(p);
-  } else {
-    e = cudaFuncSetAttribute(mlp_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SB_TOTAL);
-    if (e != cudaSuccess) return e;
-    mlp_bwd_kernel<<<grid, BWD_THREADS, SB_TOTAL, stream>>>(p);
-  }
+  const long long iters = padded_rows(p.M) / (4 * TILE_M);
+  const int pairs = num_sms / 2;
+  const int grid = int(iters < pairs ? iters : pairs) * 2;
+  cudaError_t e = cudaFuncSetAttribute(mlp_bwd_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SB_TOTAL);
+  if (e != cudaSuccess) return e;
+  mlp_bwd_pair_kernel<<<grid, BWD_THREADS, SB_TOTAL, stream>>>(p);
   return cudaGetLastError();
 }
 

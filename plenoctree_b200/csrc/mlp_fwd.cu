@@ -14,23 +14,23 @@
 //   NerfModel.eval_points_raw (models.py:143-181)       OUT_RAW / OUT_SIGMA
 //
 // Warp roles (320 threads): warps 0-3 = epilogue group 0 (tile X), warps 4-7 = epilogue group 1
-// (tile Y), warp 8 = weight producer (cp.async.bulk ring, 4 x 16 KB slots), warp 9 = MMA issuer.
-// Both tiles consume every streamed weight slot (M = 256 per weight byte), TMEM holds the two
-// 128x256 fp32 accumulators (512 columns).  NSPLIT = 3 evaluates ONE tile per iteration with
-// error-compensated fp16 operands (x = hi + lo; hi*hi + lo*hi + hi*lo), using the second tile's
-// buffers for the residual parts.
+// (tile Y), warp 8 = weight producer (cp.async.bulk ring in 64 KB of shared memory), warp 9 = MMA issuer.
+// Both tiles consume every streamed weight slot, TMEM holds the two 128x256 fp32 accumulators
+// (512 columns).
 //
-// PAIR (the default for NSPLIT = 1): two CTAs of a cluster (one TPC) run ONE tcgen05.mma.cta_group::2 stream
+// NSPLIT = 1 (fp16) runs as a CTA pair: two CTAs of a cluster (one TPC) run ONE tcgen05.mma.cta_group::2 stream
 // over FOUR tiles (512 samples per iteration).  Every MMA has M = 256 (128 rows of tile X or Y from each CTA),
 // N = 256, and reads only HALF of the weight slot from each CTA's shared memory: per CTA and MMA the operand
 // fetch drops from 12 KB to 8 KB and the weight stream from 16 KB to 8 KB per slot.  That matters because the
-// shared-memory / L1 data pipe (128 B/clk) is what the single-CTA kernel saturates: operand fetch 96 B/clk +
+// shared-memory / L1 data pipe (128 B/clk) is what a single-CTA fp16 kernel saturated: operand fetch 96 B/clk +
 // weight fill 31 B/clk during the MMA phase, before the training variant adds its 128 KB of activation stores
 // per layer step (profiles/r2_*; DESIGN.md section 6).  Only the leader CTA (cluster rank 0) issues MMAs; the
 // peer's warp 9 relays "my half-slot has landed" to the leader, the peer's epilogue warps arrive on the
 // leader's a_ready barriers through the cluster address map, and every commit is multicast to both CTAs.
-#include <cstdlib>
-
+//
+// NSPLIT = 3 (fp16x3) runs on single CTAs and evaluates ONE tile per iteration with error-compensated fp16
+// operands (x = hi + lo; hi*hi + lo*hi + hi*lo), using the second tile's buffers for the residual parts; its ring
+// holds 4 x 16 KB slots, hi and lo images in turn.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -52,7 +52,7 @@ constexpr uint32_t SM_W = SM_E1 + E_TILE_BYTES;
 constexpr uint32_t SM_TOTAL = SM_W + NUM_WSLOTS * WSLOT_BYTES;  // 229376
 static_assert(SM_TOTAL == 224 * 1024, "smem map");
 
-constexpr int MAX_RING = 8;   // pair mode: eight 8 KB half-slots in the same 64 KB
+constexpr int MAX_RING = 8;   // CTA pair: eight 8 KB half-slots in the same 64 KB
 struct Barriers {
   uint64_t full[MAX_RING];
   uint64_t empty[MAX_RING];
@@ -164,9 +164,9 @@ __device__ __forceinline__ void trace_stamp(unsigned long long* tr, int role, ui
 // OUTM (= p.out_mode) is a template parameter so that each instantiation carries only its own heads
 // epilogue: the fully unrolled 80-column heads loop with all four output modes inlined made the kernel
 // 145+ KB of SASS and cost ~8 % of inference throughput in instruction-cache misses.
-template <int NSPLIT, int OUTM, bool SAVE, bool PAIR>
+template <int NSPLIT, int OUTM, bool SAVE>
 __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
-  static_assert(!PAIR || NSPLIT == 1, "CTA pairs run the single-pass mode only");
+  constexpr bool PAIR = (NSPLIT == 1);   // the single-pass mode runs as CTA pairs, the x3 mode on single CTAs
   constexpr bool PRECISE = (NSPLIT == 3);
   __shared__ __align__(8) Barriers bars;
   __shared__ uint32_t tmem_base_s;
@@ -191,9 +191,9 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
       mbar_init(smem_u32(&bars.empty[i]), 1);
     }
     for (int g = 0; g < 2; ++g) {
-      // one arrival per epilogue warp that writes the operand tile(s) the MMA reads: 4 (own tile), 8 in the
-      // x3 mode (both groups write one tile) and in pair mode (the peer's four warps arrive remotely)
-      mbar_init(smem_u32(&bars.a_ready[g]), (NSPLIT == 1 && !PAIR) ? 4 : 8);
+      // one arrival per epilogue warp that writes the operand tile(s) the MMA reads: 8 in the x3 mode (both
+      // groups write one tile) and in pair mode (4 own warps, the peer's four arrive remotely)
+      mbar_init(smem_u32(&bars.a_ready[g]), 8);
       mbar_init(smem_u32(&bars.d_ready[g]), 1);
     }
     fence_mbar_init();
@@ -228,13 +228,9 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
           for (int part = 0; part < (NSPLIT == 3 ? 2 : 1); ++part) {
             wait_bar(&bars.empty[slot], phase ^ 1);
             if (elect_one()) {
-              if (p.debug_flags & 8) {   // timing experiment: no weight traffic at all (results are garbage)
-                mbar_arrive(smem_u32(&bars.full[slot]));
-              } else {
-                mbar_arrive_expect_tx(smem_u32(&bars.full[slot]), cbytes);
-                bulk_g2s(sbase + SM_W + slot * RSLOT_BYTES, (part == 0 ? p.w.w_hi : p.w.w_lo) + off + rank * cbytes,
-                         cbytes, smem_u32(&bars.full[slot]));
-              }
+              mbar_arrive_expect_tx(smem_u32(&bars.full[slot]), cbytes);
+              bulk_g2s(sbase + SM_W + slot * RSLOT_BYTES, (part == 0 ? p.w.w_hi : p.w.w_lo) + off + rank * cbytes,
+                       cbytes, smem_u32(&bars.full[slot]));
             }
             __syncwarp();
             if (++slot == RING) {
@@ -281,10 +277,10 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
       // so X's epilogue (accumulator drain, next operand tile) runs under Y's last turn and Y's under the first
       // turn of X's next layer — the tensor pipe no longer idles through every epilogue (lock-step tiles: 4.4 k
       // cycles of MMAs + 1.3 k of epilogue per layer).  Every weight slot is still streamed once: it stays in
-      // the ring from X's use to Y's, TURN slots later (pair mode: 5 of the 8 half-slots live, 3 of prefetch).
+      // the ring from X's use to Y's, TURN slots later (5 of the 8 half-slots live, 3 of prefetch).
       // The issue loop must average < 256 cycles per (tile, slot) = two MMAs, so everything that depends on the
       // layer structure (which tile image feeds K-slot j, bias slots, layer ends) is tabulated once per CTA.
-      constexpr int TURN = PAIR ? 5 : 2;
+      constexpr int TURN = 5;
       for (int n = int(lane); n < FWD_TRUNK_SLOTS + FWD_HEAD_SLOTS; n += 32) {
         int l = 0, j = n;
         while (l < NUM_TRUNK && j >= fwd_slots_of_layer(l)) j -= fwd_slots_of_layer(l++);
@@ -328,18 +324,11 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
                   const uint64_t bh0 = W_HI | uint64_t(w_enc0 + rs * (RSLOT_BYTES >> 4));
                   const uint32_t d = tmem + uint32_t(g) * 256u;
                   const uint32_t idesc = (e.z & 8u) ? idesc_h : idesc_t;
-                  if (PAIR) {
-                    // M = 256: rows 0-127 = this CTA's tile g, rows 128-255 = the peer's tile g (same offsets)
-                    if (!(e.z & 1u)) umma_f16_pair(d, ah0, bh0, idesc, e.z & 2u);
-                    umma_f16_pair(d, ah0 + 2, bh0 + 2, idesc, 1u);
-                    if (e.z & 4u) umma_commit_pair(smem_u32(&bars.d_ready[g]), 0x3);
-                    if (g == 1) umma_commit_pair(smem_u32(&bars.empty[rs]), 0x3);
-                  } else {
-                    if (!(e.z & 1u)) umma_f16(d, ah0, bh0, idesc, e.z & 2u);
-                    umma_f16(d, ah0 + 2, bh0 + 2, idesc, 1u);      // k16 step 1: +32 bytes = +2 encoded
-                    if (e.z & 4u) umma_commit(smem_u32(&bars.d_ready[g]));
-                    if (g == 1) umma_commit(smem_u32(&bars.empty[rs]));
-                  }
+                  // M = 256: rows 0-127 = this CTA's tile g, rows 128-255 = the peer's tile g (same offsets)
+                  if (!(e.z & 1u)) umma_f16_pair(d, ah0, bh0, idesc, e.z & 2u);
+                  umma_f16_pair(d, ah0 + 2, bh0 + 2, idesc, 1u);      // k16 step 1: +32 bytes = +2 encoded
+                  if (e.z & 4u) umma_commit_pair(smem_u32(&bars.d_ready[g]), 0x3);
+                  if (g == 1) umma_commit_pair(smem_u32(&bars.empty[rs]), 0x3);
                 }
                 __syncwarp();
                 e = en;
@@ -389,35 +378,21 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
               const uint32_t a_base = sbase + (from_e ? (g ? SM_E1 : SM_E0) : (g ? SM_A1 : SM_A0)) + a_off;
               const uint64_t ah0 = A_HI | uint64_t((a_base >> 4) & 0x3FFF);
               const uint32_t d = tmem + uint32_t(g) * 256u;
-              if (PAIR) {
-                // M = 256: rows 0-127 = this CTA's tile g, rows 128-255 = the peer's tile g (same offsets)
-                if (!bias_slot) umma_f16_pair(d, ah0, bh0, idesc, j != 0);
-                umma_f16_pair(d, ah0 + 2, bh0 + 2, idesc, 1u);
-              } else if (NSPLIT == 1) {
-                if (!bias_slot) umma_f16(d, ah0, bh0, idesc, j != 0);
-                umma_f16(d, ah0 + 2, bh0 + 2, idesc, 1u);      // k16 step 1: +32 bytes = +2 encoded
-              } else {
-                // tile 0 only: hi operand lives in the "tile 0" buffers, lo in the "tile 1" ones
-                const uint32_t a_lo_base = sbase + (from_e ? SM_E1 : SM_A1) + a_off;
-                const uint64_t al0 = A_HI | uint64_t((a_lo_base >> 4) & 0x3FFF);
-                if (!bias_slot) {
-                  umma_f16(d, al0, bh0, idesc, j != 0);
-                  umma_f16(d, ah0, bl0, idesc, 1u);
-                  umma_f16(d, ah0, bh0, idesc, 1u);
-                }
-                umma_f16(d, al0 + 2, bh0 + 2, idesc, 1u);
-                umma_f16(d, ah0 + 2, bl0 + 2, idesc, 1u);
-                umma_f16(d, ah0 + 2, bh0 + 2, idesc, 1u);
+              // tile 0 only: hi operand lives in the "tile 0" buffers, lo in the "tile 1" ones
+              const uint32_t a_lo_base = sbase + (from_e ? SM_E1 : SM_A1) + a_off;
+              const uint64_t al0 = A_HI | uint64_t((a_lo_base >> 4) & 0x3FFF);
+              if (!bias_slot) {
+                umma_f16(d, al0, bh0, idesc, j != 0);
+                umma_f16(d, ah0, bl0, idesc, 1u);
+                umma_f16(d, ah0, bh0, idesc, 1u);
               }
-              if (PAIR) {
-                if (j == ns - 1) umma_commit_pair(smem_u32(&bars.d_ready[g]), 0x3);
-                if (g == NTILES - 1) umma_commit_pair(smem_u32(&bars.empty[s_hi]), 0x3);
-              } else {
-                if (j == ns - 1) umma_commit(smem_u32(&bars.d_ready[g]));
-                if (g == NTILES - 1) {
-                  umma_commit(smem_u32(&bars.empty[s_hi]));
-                  if (NSPLIT == 3) umma_commit(smem_u32(&bars.empty[s_lo]));
-                }
+              umma_f16(d, al0 + 2, bh0 + 2, idesc, 1u);      // k16 step 1: +32 bytes = +2 encoded
+              umma_f16(d, ah0 + 2, bl0 + 2, idesc, 1u);
+              umma_f16(d, ah0 + 2, bh0 + 2, idesc, 1u);
+              if (j == ns - 1) umma_commit(smem_u32(&bars.d_ready[g]));
+              if (g == NTILES - 1) {
+                umma_commit(smem_u32(&bars.empty[s_hi]));
+                umma_commit(smem_u32(&bars.empty[s_lo]));
               }
             }
             __syncwarp();
@@ -534,9 +509,7 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
           // it, because a backed-up st.global queue blocks the warp's later st.shared / fences; a TMA bulk store of the
           // verbatim tile image (no LSU time at all) collides with the weight-slot TMA loads and with the MMA operand
           // reads: 73.5 k vs 63.1 k cycles per iteration (tried in round 2, removed).
-          // debug flag 16 (timing experiment): every h store lands in one 64 KB scratch tile per CTA (L2, not HBM)
-          uint8_t* const h_glob = p.save_h + ((p.debug_flags & 16) ? size_t(blockIdx.x)
-                                                                   : (size_t(tile_idx) * NUM_TRUNK + l)) * A_TILE_BYTES;
+          uint8_t* const h_glob = p.save_h + (size_t(tile_idx) * NUM_TRUNK + l) * A_TILE_BYTES;
           uint32_t maskw[8];
 #pragma unroll
           for (int c = 0; c < 8; ++c) {
@@ -546,12 +519,9 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
               const uint32_t unit = uint32_t((c & 1) * 4 + u);
               const uint32_t off = uint32_t(c >> 1) * A_CHUNK_BYTES + uint32_t(row) * 128u +
                                    ((unit ^ uint32_t(row & 7)) << 4);
-              uint4 q = make_uint4(off, row, c, u);
-              if (!(p.debug_flags & 256)) q = *reinterpret_cast<const uint4*>(a_hi + off);   // 256: no LDS
-              if (!(p.debug_flags & 64))   // 64: timing experiment, no h stores at all
-                *reinterpret_cast<uint4*>(h_glob + uint32_t(warp & 3) * 16384u + uint32_t(c * 4 + u) * 512u + lane * 16u) = q;
+              const uint4 q = *reinterpret_cast<const uint4*>(a_hi + off);
+              *reinterpret_cast<uint4*>(h_glob + uint32_t(warp & 3) * 16384u + uint32_t(c * 4 + u) * 512u + lane * 16u) = q;
               const uint32_t qw[4] = {q.x, q.y, q.z, q.w};
-              if (p.debug_flags & 128) { mbits ^= q.x; continue; }   // 128: no mask arithmetic
 #pragma unroll
               for (int i = 0; i < 4; ++i)   // non-negative fp16 pair -> 0/1 per half (VIMNMX.U16x2), shifted in
                 mbits = (mbits << 1) + __vminu2(qw[i], 0x00010001u);
@@ -693,37 +663,27 @@ __device__ __forceinline__ void fwd_body(const FwdParams& p, uint8_t* smem) {
   }
 }
 
+// single-CTA kernel: the x3 mode only (the single-pass mode runs as CTA pairs)
 template <int NSPLIT, int OUTM, bool SAVE>
 __global__ void __launch_bounds__(FWD_THREADS, 1)
 mlp_fwd_kernel(const __grid_constant__ FwdParams p) {
+  static_assert(NSPLIT == 3 && !SAVE, "single-CTA kernel: x3 inference only");
   extern __shared__ __align__(1024) uint8_t smem[];
-  fwd_body<NSPLIT, OUTM, SAVE, false>(p, smem);
+  fwd_body<NSPLIT, OUTM, SAVE>(p, smem);
 }
 
 template <int OUTM, bool SAVE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(FWD_THREADS, 1)
 mlp_fwd_pair_kernel(const __grid_constant__ FwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
-  fwd_body<1, OUTM, SAVE, true>(p, smem);
+  fwd_body<1, OUTM, SAVE>(p, smem);
 }
 
-// POB_PAIR=0 selects the single-CTA kernels for the single-pass mode (A/B experiments; default: CTA pairs)
-bool pair_mode_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("POB_PAIR");
-    v = e ? atoi(e) : 1;
-  }
-  return v != 0;
-}
-
-cudaError_t launch_mlp_fwd(const FwdParams& p, int nsplit, bool precise_sin, int num_sms,
-                           cudaStream_t stream) {
+cudaError_t launch_mlp_fwd(const FwdParams& p, int nsplit, int num_sms, cudaStream_t stream) {
   if (p.M <= 0) return cudaSuccess;
-  (void)precise_sin;   // tied to the precision mode: FP16X3 uses libdevice sinf, FP16 the reduced SFU sine
   if (nsplit != 1 && nsplit != 3) return cudaErrorInvalidValue;
-  const bool pair = nsplit == 1 && num_sms >= 2 && pair_mode_enabled();
-  const int rows = pair ? 4 * TILE_M : ((nsplit == 1) ? 2 * TILE_M : TILE_M);
+  const bool pair = nsplit == 1;
+  const int rows = pair ? 4 * TILE_M : TILE_M;
   const long long iters = (p.M + rows - 1) / rows;
   const int units = pair ? num_sms / 2 : num_sms;
   const int grid = int(iters < units ? iters : units) * (pair ? 2 : 1);
@@ -748,19 +708,11 @@ cudaError_t launch_mlp_fwd(const FwdParams& p, int nsplit, bool precise_sin, int
     }
   }
   switch (p.out_mode) {
-    case OUT_RAW:
-      return nsplit == 1 ? launch(mlp_fwd_kernel<1, OUT_RAW, false>) : launch(mlp_fwd_kernel<3, OUT_RAW, false>);
-    case OUT_SIGMA:
-      if (save) return launch(mlp_fwd_kernel<1, OUT_SIGMA, true>);
-      return nsplit == 1 ? launch(mlp_fwd_kernel<1, OUT_SIGMA, false>) : launch(mlp_fwd_kernel<3, OUT_SIGMA, false>);
-    case OUT_RGBS:
-      if (save) return launch(mlp_fwd_kernel<1, OUT_RGBS, true>);
-      return nsplit == 1 ? launch(mlp_fwd_kernel<1, OUT_RGBS, false>) : launch(mlp_fwd_kernel<3, OUT_RGBS, false>);
-    case OUT_CELL_MEAN:
-      return nsplit == 1 ? launch(mlp_fwd_kernel<1, OUT_CELL_MEAN, false>)
-                         : launch(mlp_fwd_kernel<3, OUT_CELL_MEAN, false>);
-    default:
-      return cudaErrorInvalidValue;
+    case OUT_RAW: return launch(mlp_fwd_kernel<3, OUT_RAW, false>);
+    case OUT_SIGMA: return launch(mlp_fwd_kernel<3, OUT_SIGMA, false>);
+    case OUT_RGBS: return launch(mlp_fwd_kernel<3, OUT_RGBS, false>);
+    case OUT_CELL_MEAN: return launch(mlp_fwd_kernel<3, OUT_CELL_MEAN, false>);
+    default: return cudaErrorInvalidValue;
   }
 }
 

@@ -10,14 +10,12 @@
 // products, exp, sigmoid, compositing sums) may contract to FMA and uses the fast exp / reciprocal — the march is
 // instruction-issue bound (ncu: sm__throughput 73-79 %, DRAM 5 %), so instruction count is what matters.
 //
-// Thread mapping (B200-first, not svox's thread-per-ray): a *group* of G lanes owns one ray (G = 4 by default,
-// see group_width(); 8 / 16 / 32 selectable for profiling).  All lanes of a group walk the tree together
-// (same-address loads broadcast), lane l owns basis functions l, l+G, ...: the 3K coefficient gather of a
-// contributing leaf is three coalesced segments per group instead of 3K strided scalar loads per thread, the dot
-// products finish with log2(G) shuffles, and the backward scatter issues coalesced RED.ADD.F32.  Pixels are tiled
-// per CTA so that neighbouring rays share L1 lines.
+// Thread mapping (B200-first, not svox's thread-per-ray): a *group* of G = 4 lanes owns one ray (see G below).
+// All lanes of a group walk the tree together (same-address loads broadcast), lane l owns basis functions l, l+G,
+// ...: the 3K coefficient gather of a contributing leaf is three coalesced segments per group instead of 3K
+// strided scalar loads per thread, the dot products finish with log2(G) shuffles, and the backward scatter issues
+// coalesced RED.ADD.F32.  Pixels are tiled per CTA so that neighbouring rays share L1 lines.
 #include <cstdint>
-#include <cstdlib>
 
 #include "../../include/plenoctree_b200.h"
 #include "capi_util.h"
@@ -32,6 +30,14 @@ namespace {
 // (renderer_step_size 1e-5, octree/config/syn_sh16.json:16,22,24), since every iteration advances by >= step_size.
 constexpr int MAX_MARCH_STEPS = 1 << 20;
 constexpr int MAX_TREE_DEPTH = 40;
+
+// Lanes per ray (group width G).  The march is instruction-issue bound and every lane of a group repeats the walk,
+// so fewer lanes per ray = fewer instructions per ray.  Measured 800x800 / depth-8 SH16: 16 lanes 4.1 ms, 8 lanes
+// 2.25 ms, 4 lanes 1.65 ms.  (2 lanes: 1.52 ms render but 4.7 ms training pass — not kept.)
+constexpr int G = 4;
+constexpr int RAYS_PER_CTA = 256 / G;
+// perspective camera: each CTA renders an 8 x 8 pixel tile
+constexpr int PIX_TILE_W = 8, PIX_TILE_H = RAYS_PER_CTA / PIX_TILE_W;
 
 struct TreeDev {
   const float* data;
@@ -141,14 +147,11 @@ __device__ __forceinline__ long long query_leaf(const int32_t* __restrict__ chil
   return idx;
 }
 
-template <int G>
 __device__ __forceinline__ unsigned group_mask() {
-  if (G == 32) return 0xffffffffu;
   const unsigned lane = threadIdx.x & 31;
   return ((1u << G) - 1u) << (lane / G * G);
 }
 
-template <int G>
 __device__ __forceinline__ float group_sum(float v, unsigned mask) {
 #pragma unroll
   for (int s = G / 2; s > 0; s >>= 1) v += __shfl_xor_sync(mask, v, s, G);
@@ -165,10 +168,9 @@ __device__ __forceinline__ float sigmoidf(float x) { return __fdividef(1.0f, 1.0
 // idle lanes are the stack), the shared depth is a count-leading-zeros of the XOR of the integer coordinates, and
 // the position inside the leaf is frac(x * 2^(depth+1)) — bit-identical to the iterated form.  Other branch
 // factors, and levels deeper than 22, use the plain walk.
-template <int G>
 struct Marcher {
   unsigned pq0, pq1, pq2;
-  static constexpr int PW = G >= 8 ? 1 : 8 / G;   // path registers per lane: levels l, l+G, ... are cached
+  static constexpr int PW = 8 / G;   // path registers per lane: levels l, l+G, ... are cached
   static constexpr int CACHED = G * PW;
   int pdepth;     // depth of the previous leaf, -1 = no previous sample
   int path[PW];   // lane l, register j: node entered at level l + j*G (level 0: root)
@@ -278,7 +280,7 @@ struct Marcher {
 // ---- forward march of one ray by one lane group -------------------------------------------------------
 // Software-pipelined: the loads of the current leaf (sigma and this lane's three coefficients, issued
 // unconditionally) are in flight while the next leaf is located; the march itself never depends on the data.
-template <int G, int KPL>
+template <int KPL>
 __device__ __forceinline__ void trace_forward(const TreeDev& T, const Opts& O, const Ray& r, const float* basis_l, int l,
                                               unsigned mask, float* out, unsigned& visits, unsigned& hits) {
   if (!r.hit) {
@@ -293,7 +295,7 @@ __device__ __forceinline__ void trace_forward(const TreeDev& T, const Opts& O, c
     out[0] = out[1] = out[2] = O.bg;  // light = 1
     return;
   }
-  Marcher<G> m;
+  Marcher m;
   m.init();
   float delta_t;
   unsigned idx = m.locate(T, r, O.step, t, l, mask, delta_t);
@@ -328,9 +330,9 @@ __device__ __forceinline__ void trace_forward(const TreeDev& T, const Opts& O, c
         p1 += basis_l[j] * c1[j];
         p2 += basis_l[j] * c2[j];
       }
-      p0 = group_sum<G>(p0, mask);
-      p1 = group_sum<G>(p1, mask);
-      p2 = group_sum<G>(p2, mask);
+      p0 = group_sum(p0, mask);
+      p1 = group_sum(p1, mask);
+      p2 = group_sum(p2, mask);
       out[0] += weight * sigmoidf(p0);
       out[1] += weight * sigmoidf(p1);
       out[2] += weight * sigmoidf(p2);
@@ -356,7 +358,7 @@ __device__ __forceinline__ void trace_forward(const TreeDev& T, const Opts& O, c
 // ---- backward march: colour and density gradients in one pass ---------------------------------------
 // accum enters as sum_j w_j (c_j . g) + T_end * bg * sum(g) = g . out (svox computes it with an extra march:
 // trace_ray_backward pass 1); every contributing leaf then peels its own term off.
-template <int G, int KPL>
+template <int KPL>
 __device__ __forceinline__ void trace_backward(const TreeDev& T, const Opts& O, const Ray& r, const float* basis_l, int l,
                                                unsigned mask, const float* g, float accum,
                                                float* __restrict__ grad) {
@@ -365,7 +367,7 @@ __device__ __forceinline__ void trace_backward(const TreeDev& T, const Opts& O, 
   float t = r.tmin;
   const int K = T.K, D = T.D;
   if (!(t < r.tmax)) return;
-  Marcher<G> m;
+  Marcher m;
   m.init();
   float delta_t;
   unsigned idx = m.locate(T, r, O.step, t, l, mask, delta_t);
@@ -398,9 +400,9 @@ __device__ __forceinline__ void trace_backward(const TreeDev& T, const Opts& O, 
         p1 += basis_l[j] * c1[j];
         p2 += basis_l[j] * c2[j];
       }
-      p0 = group_sum<G>(p0, mask);
-      p1 = group_sum<G>(p1, mask);
-      p2 = group_sum<G>(p2, mask);
+      p0 = group_sum(p0, mask);
+      p1 = group_sum(p1, mask);
+      p2 = group_sum(p2, mask);
       const float s0 = sigmoidf(p0), s1 = sigmoidf(p1), s2 = sigmoidf(p2);
       float* gv = grad + size_t(idx) * unsigned(D);
       const float t0 = weight * s0 * (1.0f - s0) * g[0];
@@ -428,13 +430,11 @@ __device__ __forceinline__ void trace_backward(const TreeDev& T, const Opts& O, 
 }
 
 // ---- ray fetch: lane group -> ray index (pixel tiles for the perspective camera) --------------------------
-template <int G>
 __device__ __forceinline__ bool fetch_ray(const RaySrc& S, const TreeDev& T, Ray& r, long long& out_index) {
-  constexpr int RPB = 256 / G;  // rays per CTA
   const int grp = threadIdx.x / G;
   float o[3], d[3];
   if (S.o != nullptr) {
-    const long long i = (long long)blockIdx.x * RPB + grp;
+    const long long i = (long long)blockIdx.x * RAYS_PER_CTA + grp;
     if (i >= S.n) return false;
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
@@ -446,12 +446,11 @@ __device__ __forceinline__ bool fetch_ray(const RaySrc& S, const TreeDev& T, Ray
     out_index = i;
     return true;
   }
-  constexpr int TW = RPB >= 64 ? 8 : 4, TH = RPB / TW;
   const int W = int(S.cam.width);
-  const int tiles_x = (W + TW - 1) / TW;
+  const int tiles_x = (W + PIX_TILE_W - 1) / PIX_TILE_W;
   const int tx = blockIdx.x % tiles_x, ty = blockIdx.x / tiles_x;
-  const int ix = tx * TW + grp % TW;
-  const int iyl = ty * TH + grp / TW;  // row inside the slab
+  const int ix = tx * PIX_TILE_W + grp % PIX_TILE_W;
+  const int iyl = ty * PIX_TILE_H + grp / PIX_TILE_W;  // row inside the slab
   if (ix >= W || iyl >= S.nrows) return false;
   cam_ray(S.cam, ix, S.row0 + iyl, o, d);
   setup_ray(T.off, T.inv, o, d, d, r);
@@ -459,7 +458,7 @@ __device__ __forceinline__ bool fetch_ray(const RaySrc& S, const TreeDev& T, Ray
   return true;
 }
 
-template <int G, int KPL>
+template <int KPL>
 __device__ __forceinline__ void lane_basis(const TreeDev& T, const Ray& r, int l, float* bl) {
   if (T.rgba) {
 #pragma unroll
@@ -480,19 +479,22 @@ __device__ __forceinline__ void lane_basis(const TreeDev& T, const Ray& r, int l
   }
 }
 
-template <int G, int KPL>
+// The kernels keep the group width as their first template argument (always G), so that their names
+// (octree_render_kernel<4, KPL>, ...) stay those of the recorded profiles.  KPL = basis functions per lane.
+template <int GW, int KPL>
 __global__ void __launch_bounds__(256) octree_render_kernel(TreeDev T, Opts O, RaySrc S, float* __restrict__ out_rgb,
                                                             unsigned long long* __restrict__ counters) {
+  static_assert(GW == G, "one group width");
   Ray r;
   long long oi;
-  if (!fetch_ray<G>(S, T, r, oi)) return;
+  if (!fetch_ray(S, T, r, oi)) return;
   const int l = threadIdx.x % G;
-  const unsigned mask = group_mask<G>();
+  const unsigned mask = group_mask();
   float bl[KPL];
-  lane_basis<G, KPL>(T, r, l, bl);
+  lane_basis<KPL>(T, r, l, bl);
   float out[3];
   unsigned visits = 0, hits = 0;
-  trace_forward<G, KPL>(T, O, r, bl, l, mask, out, visits, hits);
+  trace_forward<KPL>(T, O, r, bl, l, mask, out, visits, hits);
   if (l < 3) out_rgb[3 * oi + l] = l == 0 ? out[0] : l == 1 ? out[1] : out[2];
   if (counters != nullptr && l == 0) {
     atomicAdd(counters + 0, (unsigned long long)visits);
@@ -501,48 +503,50 @@ __global__ void __launch_bounds__(256) octree_render_kernel(TreeDev T, Opts O, R
 }
 
 // VolumeRenderer backward for an upstream gradient d loss / d rgb  (svox trace_ray_backward)
-template <int G, int KPL>
+template <int GW, int KPL>
 __global__ void __launch_bounds__(256) octree_backward_kernel(TreeDev T, Opts O, RaySrc S,
                                                               const float* __restrict__ grad_out,
                                                               float* __restrict__ grad_data) {
+  static_assert(GW == G, "one group width");
   Ray r;
   long long oi;
-  if (!fetch_ray<G>(S, T, r, oi)) return;
+  if (!fetch_ray(S, T, r, oi)) return;
   const int l = threadIdx.x % G;
-  const unsigned mask = group_mask<G>();
+  const unsigned mask = group_mask();
   float bl[KPL];
-  lane_basis<G, KPL>(T, r, l, bl);
+  lane_basis<KPL>(T, r, l, bl);
   float out[3];
   unsigned visits = 0, hits = 0;
   Opts Of = O;
   Of.sigma_thresh = 0.f;
   Of.stop_thresh = 0.f;
-  trace_forward<G, KPL>(T, Of, r, bl, l, mask, out, visits, hits);
+  trace_forward<KPL>(T, Of, r, bl, l, mask, out, visits, hits);
   float g[3] = {__ldg(grad_out + 3 * oi), __ldg(grad_out + 3 * oi + 1), __ldg(grad_out + 3 * oi + 2)};
   const float accum = g[0] * out[0] + g[1] * out[1] + g[2] * out[2];
-  trace_backward<G, KPL>(T, Of, r, bl, l, mask, g, accum, grad_data);
+  trace_backward<KPL>(T, Of, r, bl, l, mask, g, accum, grad_data);
 }
 
 // One training pass over a camera slab (octree/optimization.py:201-207 minus the optimiser):
 //   im = render_persp(c2w); mse = mean((clamp(im,0,1) - gt)^2); mse.backward()
 // g = grad_scale * 2 * (clamp(im) - gt) inside the clamp range, 0 outside (torch.clamp's gradient).
-template <int G, int KPL>
+template <int GW, int KPL>
 __global__ void __launch_bounds__(256) octree_train_kernel(TreeDev T, Opts O, RaySrc S, const float* __restrict__ gt,
                                                            float grad_scale, float* __restrict__ grad_data,
                                                            double* __restrict__ sq_err_sum,
                                                            float* __restrict__ out_rgb) {
+  static_assert(GW == G, "one group width");
   Ray r;
   long long oi;
-  const bool have = fetch_ray<G>(S, T, r, oi);
+  const bool have = fetch_ray(S, T, r, oi);
   float err = 0.f;
   if (have) {
     const int l = threadIdx.x % G;
-    const unsigned mask = group_mask<G>();
+    const unsigned mask = group_mask();
     float bl[KPL];
-    lane_basis<G, KPL>(T, r, l, bl);
+    lane_basis<KPL>(T, r, l, bl);
     float out[3];
     unsigned visits = 0, hits = 0;
-    trace_forward<G, KPL>(T, O, r, bl, l, mask, out, visits, hits);
+    trace_forward<KPL>(T, O, r, bl, l, mask, out, visits, hits);
     float g[3];
     float accum = 0.f;
 #pragma unroll
@@ -554,7 +558,7 @@ __global__ void __launch_bounds__(256) octree_train_kernel(TreeDev T, Opts O, Ra
       accum += g[c] * out[c];
     }
     if (out_rgb != nullptr && l < 3) out_rgb[3 * oi + l] = l == 0 ? out[0] : l == 1 ? out[1] : out[2];
-    if (g[0] != 0.f || g[1] != 0.f || g[2] != 0.f) trace_backward<G, KPL>(T, O, r, bl, l, mask, g, accum, grad_data);
+    if (g[0] != 0.f || g[1] != 0.f || g[2] != 0.f) trace_backward<KPL>(T, O, r, bl, l, mask, g, accum, grad_data);
     if (l != 0) err = 0.f;
   }
   // CTA reduction of the squared error (one double atomic per CTA)
@@ -722,39 +726,17 @@ int opts_dev(const char* where, const pob_octree_opts* o, Opts& O) {
   return 0;
 }
 
-// Group width / coefficients per lane.  Default: 4 lanes per ray (the march is instruction-issue bound and every
-// lane of a group repeats the walk, so fewer lanes per ray = fewer instructions per ray; lane l owns basis functions
-// l, l+4, ...).  Measured 800x800 / depth-8 SH16: 16 lanes 4.1 ms, 8 lanes 2.25 ms, 4 lanes 1.65 ms.
-// (2 lanes: 1.52 ms render but 4.7 ms training pass — not kept.)  POB_OCTREE_G=8|16|32 selects the other
-// mappings (profiling).
-int group_width(int K) {
-  static int env = -1;
-  if (env < 0) {
-    const char* e = getenv("POB_OCTREE_G");
-    env = e ? atoi(e) : 0;
-  }
-  if (env == 32) return 32;
-  if (env == 16) return K > 16 ? 32 : 16;
-  if (env == 8) return 8;
-  return 4;
-}
-
-#define POB_OCTREE_DISPATCH(KERNEL, G, K, ...)                                   \
+// basis functions per lane: K = 1 or 4 -> 1, 9 -> 3, 16 -> 4, 25 -> 7
+#define POB_OCTREE_DISPATCH(KERNEL, K, ...)                                      \
   do {                                                                           \
-    if ((G) == 32) KERNEL<32, 1><<<blocks, 256, 0, st>>>(__VA_ARGS__);           \
-    else if ((G) == 16) KERNEL<16, 1><<<blocks, 256, 0, st>>>(__VA_ARGS__);      \
-    else if ((G) == 4 && (K) <= 4) KERNEL<4, 1><<<blocks, 256, 0, st>>>(__VA_ARGS__);   \
-    else if ((G) == 4 && (K) <= 12) KERNEL<4, 3><<<blocks, 256, 0, st>>>(__VA_ARGS__);  \
-    else if ((G) == 4 && (K) <= 16) KERNEL<4, 4><<<blocks, 256, 0, st>>>(__VA_ARGS__);  \
-    else if ((G) == 4) KERNEL<4, 7><<<blocks, 256, 0, st>>>(__VA_ARGS__);               \
-    else if ((K) <= 8) KERNEL<8, 1><<<blocks, 256, 0, st>>>(__VA_ARGS__);        \
-    else if ((K) <= 16) KERNEL<8, 2><<<blocks, 256, 0, st>>>(__VA_ARGS__);       \
-    else KERNEL<8, 4><<<blocks, 256, 0, st>>>(__VA_ARGS__);                      \
+    if ((K) <= 4) KERNEL<G, 1><<<blocks, 256, 0, st>>>(__VA_ARGS__);             \
+    else if ((K) <= 12) KERNEL<G, 3><<<blocks, 256, 0, st>>>(__VA_ARGS__);       \
+    else if ((K) <= 16) KERNEL<G, 4><<<blocks, 256, 0, st>>>(__VA_ARGS__);       \
+    else KERNEL<G, 7><<<blocks, 256, 0, st>>>(__VA_ARGS__);                      \
   } while (0)
 
 int ray_src(const char* where, const float* o, const float* d, const float* v, long long n, const pob_camera* cam,
-            int row0, int nrows, RaySrc& S, unsigned& blocks, int G) {
-  const int rpb = 256 / G;
+            int row0, int nrows, RaySrc& S, unsigned& blocks) {
   S.o = o;
   S.d = d;
   S.v = v;
@@ -764,7 +746,7 @@ int ray_src(const char* where, const float* o, const float* d, const float* v, l
   if (cam == nullptr) {
     if (!o || !d || !v) return pob_fail(where, "ray pointers are NULL");
     if (n < 0) return pob_fail(where, "negative ray count");
-    blocks = unsigned((n + rpb - 1) / rpb);
+    blocks = unsigned((n + RAYS_PER_CTA - 1) / RAYS_PER_CTA);
     return 0;
   }
   S.o = S.d = S.v = nullptr;
@@ -779,8 +761,7 @@ int ray_src(const char* where, const float* o, const float* d, const float* v, l
   S.row0 = row0;
   S.nrows = nrows;
   S.n = (long long)nrows * W;
-  const int tw = rpb >= 64 ? 8 : 4, th = rpb / tw;
-  blocks = unsigned(((W + tw - 1) / tw) * ((nrows + th - 1) / th));
+  blocks = unsigned(((W + PIX_TILE_W - 1) / PIX_TILE_W) * ((nrows + PIX_TILE_H - 1) / PIX_TILE_H));
   return 0;
 }
 
@@ -798,13 +779,12 @@ int pob_octree_render(const pob_octree* tree, const pob_octree_opts* opts, const
   unsigned blocks = 0;
   if (int rc = tree_dev(W, tree, T)) return rc;
   if (int rc = opts_dev(W, opts, O)) return rc;
-  const int G = group_width(T.K);
-  if (int rc = ray_src(W, origins_dev, dirs_dev, vdirs_dev, n_rays, cam, row0, nrows, S, blocks, G)) return rc;
+  if (int rc = ray_src(W, origins_dev, dirs_dev, vdirs_dev, n_rays, cam, row0, nrows, S, blocks)) return rc;
   if (!out_rgb_dev) return pob_fail(W, "output pointer is NULL");
   if (blocks == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   pob_count_launch();
-  POB_OCTREE_DISPATCH(octree_render_kernel, G, T.K, T, O, S, out_rgb_dev, counters_dev);
+  POB_OCTREE_DISPATCH(octree_render_kernel, T.K, T, O, S, out_rgb_dev, counters_dev);
   POB_CUDA(W, cudaGetLastError());
   return 0;
 }
@@ -819,13 +799,12 @@ int pob_octree_render_backward(const pob_octree* tree, const pob_octree_opts* op
   unsigned blocks = 0;
   if (int rc = tree_dev(W, tree, T)) return rc;
   if (int rc = opts_dev(W, opts, O)) return rc;
-  const int G = group_width(T.K);
-  if (int rc = ray_src(W, origins_dev, dirs_dev, vdirs_dev, n_rays, cam, row0, nrows, S, blocks, G)) return rc;
+  if (int rc = ray_src(W, origins_dev, dirs_dev, vdirs_dev, n_rays, cam, row0, nrows, S, blocks)) return rc;
   if (!grad_out_dev || !grad_data_dev) return pob_fail(W, "gradient pointer is NULL");
   if (blocks == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   pob_count_launch();
-  POB_OCTREE_DISPATCH(octree_backward_kernel, G, T.K, T, O, S, grad_out_dev, grad_data_dev);
+  POB_OCTREE_DISPATCH(octree_backward_kernel, T.K, T, O, S, grad_out_dev, grad_data_dev);
   POB_CUDA(W, cudaGetLastError());
   return 0;
 }
@@ -843,13 +822,12 @@ int pob_octree_train_persp(const pob_octree* tree, const pob_octree_opts* opts, 
   if (!cam) return pob_fail(W, "camera is NULL");
   if (O.sigma_thresh != 0.f || O.stop_thresh != 0.f)
     return pob_fail(W, "training renders with sigma_thresh = stop_thresh = 0 (svox fast=False)");
-  const int G = group_width(T.K);
-  if (int rc = ray_src(W, nullptr, nullptr, nullptr, 0, cam, row0, nrows, S, blocks, G)) return rc;
+  if (int rc = ray_src(W, nullptr, nullptr, nullptr, 0, cam, row0, nrows, S, blocks)) return rc;
   if (!gt_rgb_dev || !grad_data_dev) return pob_fail(W, "gt / gradient pointer is NULL");
   if (blocks == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   pob_count_launch();
-  POB_OCTREE_DISPATCH(octree_train_kernel, G, T.K, T, O, S, gt_rgb_dev, grad_scale, grad_data_dev, sq_err_sum_dev,
+  POB_OCTREE_DISPATCH(octree_train_kernel, T.K, T, O, S, gt_rgb_dev, grad_scale, grad_data_dev, sq_err_sum_dev,
                       out_rgb_dev);
   POB_CUDA(W, cudaGetLastError());
   return 0;

@@ -133,7 +133,7 @@ int forward_levels(const char* where, const pob_render_config& c, Workspace& w, 
       p.save_e = C.E;
       p.save_mask = C.mask;
     }
-    { pob_count_launch(1); PobPhaseTimer _t(POB_PH_FWD, st); POB_CUDA(where, launch_mlp_fwd(p, precision, precision == POB_PREC_FP16X3, sms, st)); }
+    { pob_count_launch(1); PobPhaseTimer _t(POB_PH_FWD, st); POB_CUDA(where, launch_mlp_fwd(p, precision, sms, st)); }
   }
   { pob_count_launch(1); PobPhaseTimer _t(POB_PH_RENDER, st); POB_CUDA(where, launch_composite_fwd(C.rgbs, C.z, d, R, Nc, c.white_bkgd, C.comp, C.disp, C.acc, C.weights, st)); }
   if (Nf > 0) {
@@ -154,7 +154,7 @@ int forward_levels(const char* where, const pob_render_config& c, Workspace& w, 
       p.save_e = F.E;
       p.save_mask = F.mask;
     }
-    { pob_count_launch(1); PobPhaseTimer _t(POB_PH_FWD, st); POB_CUDA(where, launch_mlp_fwd(p, precision, precision == POB_PREC_FP16X3, sms, st)); }
+    { pob_count_launch(1); PobPhaseTimer _t(POB_PH_FWD, st); POB_CUDA(where, launch_mlp_fwd(p, precision, sms, st)); }
     { pob_count_launch(1); PobPhaseTimer _t(POB_PH_RENDER, st); POB_CUDA(where, launch_composite_fwd(F.rgbs, F.z, d, R, Nc + Nf, c.white_bkgd, F.comp, F.disp, F.acc,
                                          F.weights, st)); }
   }
@@ -214,7 +214,7 @@ int pob_loss_and_grad(const pob_render_config* cfg, const pob_train_hparams* hp,
                       const float* viewdirs_dev, const float* pixels_dev, int n_rays, const float* z_base_dev,
                       const float* t_rand_dev, const float* u_dev, int u_per_ray, const float* z_fine_dev,
                       const float* sp_points_dev, float* grad_flat_dev, float* stats_dev, void* workspace_dev,
-                      void* mlp0_done_event, void* stream) {
+                      void* stream) {
   const char* where = "pob_loss_and_grad";
   if (int e = check_cfg(where, cfg)) return e;
   if (!hp) return pob_fail(where, "hparams is NULL");
@@ -259,9 +259,8 @@ int pob_loss_and_grad(const pob_render_config* cfg, const pob_train_hparams* hp,
                                                                                                     LAST.G + Mr_last, stats_dev + 2, st)); }
   }
   // ---- backward: per MLP one dgrad launch, then ONE wgrad launch over its saved dZ / h tiles ----
-  // MLP_0 (coarse level only) is finished first: its branch of the graph is independent of MLP_1's
-  // (stop_gradient, model_utils.py:286), so the caller can all-reduce the MLP_0 bucket of the gradient
-  // (mlp0_done_event) while the 3x larger MLP_1 backward is still running.
+  // MLP_0 (coarse level only) first: its branch of the graph is independent of MLP_1's (stop_gradient,
+  // model_utils.py:286), so grad_flat[0 : P) is final before the 3x larger MLP_1 backward starts.
   const int NH = heads_width(K);
   for (int mlp = 0; mlp < (Nf > 0 ? 2 : 1); ++mlp) {
     Level& L = mlp == 0 ? C : F;
@@ -295,7 +294,6 @@ int pob_loss_and_grad(const pob_render_config* cfg, const pob_train_hparams* hp,
     { pob_count_launch(); PobPhaseTimer _t(POB_PH_WGRAD, st); POB_CUDA(where, launch_mlp_wgrad(g, nctas, st)); }
     { pob_count_launch(); PobPhaseTimer _t(POB_PH_OPTIM, st); POB_CUDA(where, launch_reduce_grads(w.partials[mlp], rs, rc, K, 1.0f / hp->loss_scale,
                                         grad_flat_dev + size_t(mlp) * P, st)); }
-    if (mlp == 0 && Nf > 0 && mlp0_done_event) POB_CUDA(where, cudaEventRecord((cudaEvent_t)mlp0_done_event, st));
   }
   return 0;
 }

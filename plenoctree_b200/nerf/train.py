@@ -1,8 +1,7 @@
 """train_step of the reference (nerf_sh/train.py:51-121) on the CUDA library.
 
     loss_fn + value_and_grad   -> lib.pob_loss_and_grad   (fused tcgen05 forward / dgrad / wgrad)
-    lax.pmean(grad, "batch")   -> two torch.distributed all-reduces on the flat gradient (NCCL): the MLP_0 bucket
-                                  on a side stream while the MLP_1 backward still runs, then [MLP_1 | stats]
+    lax.pmean(grad, "batch")   -> one torch.distributed all-reduce (NCCL) on the flat [gradient | stats] buffer
     optimizer.apply_gradient   -> lib.pob_adam_update      (flax Adam + operand re-pack)
 GraphedTrainStep captures the whole step (jitter draws, kernels, collectives, Adam) in one CUDA graph.
 
@@ -46,12 +45,9 @@ class TrainState:
         self.step = 0
         # gradient buffer: [params | 8 stats] so that the last all-reduce carries both pmean calls
         self.gbuf = torch.zeros(model.params.numel() + 8, dtype=torch.float32, device=model.device)
-        # device copy of (lr, step) for replayable graphs, bucket-overlap plumbing (created on first use)
+        # device copy of (lr, step) for replayable graphs
         self.lr_step = torch.zeros(2, dtype=torch.float32, device=model.device)
         self.rng_seed = 20200823 + 7919 * (dist.get_rank() if dist.is_available() and dist.is_initialized() else 0)
-        self.side_stream = None
-        self.ev_mlp0 = None
-        self.ev_bucket0 = None
 
     @property
     def grads(self):
@@ -69,9 +65,8 @@ def default_loss_scale(n_rays):
 
 def loss_and_grad(model, state, batch, sparsity_weight=1e-3, sparsity_length=0.05, sparsity_radius=1.5,
                   randomized=True, t_rand=None, u=None, sp_points=None, loss_scale=None, z_fine=None,
-                  sigma_noise=None, mlp0_event=None, lr_step_on_device=False):
-    """value_and_grad(loss_fn) for this rank's shard; fills state.grads / state.stats_raw (device).
-    mlp0_event (torch.cuda.Event): recorded on the current stream once the MLP_0 half of the gradient is final."""
+                  sigma_noise=None, lr_step_on_device=False):
+    """value_and_grad(loss_fn) for this rank's shard; fills state.grads / state.stats_raw (device)."""
     rays = batch["rays"]
     o = _cuda_f32(rays.origins, "rays.origins", 3)
     d = _cuda_f32(rays.directions, "rays.directions", 3)
@@ -99,8 +94,7 @@ def loss_and_grad(model, state, batch, sparsity_weight=1e-3, sparsity_length=0.0
                                 ptr(model.blobs[1]) if model.num_mlps == 2 else None, ptr(o), ptr(d), ptr(v),
                                 ptr(px), n, ptr(model.z_base), ptr(t_rand), ptr(u), upr,
                                 ptr(z_fine), ptr(sp_points) if use_sp else None, ptr(state.grads),
-                                ptr(state.stats_raw), ptr(ws),
-                                mlp0_event.cuda_event if mlp0_event is not None else None, stream_ptr()))
+                                ptr(state.stats_raw), ptr(ws), stream_ptr()))
     return n
 
 
@@ -148,25 +142,6 @@ def allreduce_gradients(gbuf):
     return world
 
 
-def bucket_overlap_enabled():
-    """POB_BUCKET_OVERLAP=1: all-reduce the MLP_0 half of the gradient on a side stream under the MLP_1 backward.
-    Off by default: the forward / backward kernels are persistent, one CTA (pair) per SM with a static share of
-    the tiles, so the SMs an overlapping NCCL kernel occupies start their share late and the launch ends later by
-    about the time the overlap saved (measured at 2 GPUs: bench_extras `strong`, DESIGN.md section 7)."""
-    import os
-    return os.environ.get("POB_BUCKET_OVERLAP", "0") not in ("", "0")
-
-
-def _bucket_plumbing(state):
-    if state.side_stream is None:
-        state.side_stream = torch.cuda.Stream(device=state.model.device)
-        state.ev_mlp0 = torch.cuda.Event()
-        state.ev_bucket0 = torch.cuda.Event()
-        state.ev_mlp0.record()          # materialise the cudaEvent_t handles
-        state.ev_bucket0.record()
-    return state.side_stream, state.ev_mlp0, state.ev_bucket0
-
-
 def shard_batch(batch_size, rank, world):
     """reference semantics: batch_size is global and split evenly over devices (utils.py:518-522,252)."""
     if batch_size % world != 0:
@@ -181,24 +156,10 @@ def train_step(model, state, batch, lr, sparsity_weight=1e-3, sparsity_length=0.
     """One optimisation step (nerf_sh/train.py:51-121).  Returns Stats when sync_stats (forces a
     device->host read of the six scalars, like the reference's periodic logging), else None."""
     world = _world() if collective else 1     # collective=False: single-rank semantics inside a multi-rank job
-    P = model.P
-    if world > 1 and model.num_mlps == 2 and bucket_overlap_enabled():
-        # two buckets: MLP_0's half is all-reduced on a side stream as soon as its backward is done (the event is
-        # recorded inside pob_loss_and_grad), hidden under the MLP_1 backward; [MLP_1 | stats] follows on this stream
-        side, ev_mlp0, ev_b0 = _bucket_plumbing(state)
-        n = loss_and_grad(model, state, batch, sparsity_weight, sparsity_length, sparsity_radius, randomized, t_rand,
-                          u, sp_points, loss_scale, mlp0_event=ev_mlp0, lr_step_on_device=lr_step_on_device)
-        side.wait_event(ev_mlp0)
-        with torch.cuda.stream(side):
-            dist.all_reduce(state.gbuf[:P], op=dist.ReduceOp.SUM)
-            ev_b0.record(side)
-        dist.all_reduce(state.gbuf[P:], op=dist.ReduceOp.SUM)
-        torch.cuda.current_stream().wait_event(ev_b0)
-    else:
-        n = loss_and_grad(model, state, batch, sparsity_weight, sparsity_length, sparsity_radius, randomized, t_rand,
-                          u, sp_points, loss_scale, lr_step_on_device=lr_step_on_device)
-        if world > 1:
-            allreduce_gradients(state.gbuf)   # pmean(grad) and pmean(stats) in one bucket
+    n = loss_and_grad(model, state, batch, sparsity_weight, sparsity_length, sparsity_radius, randomized, t_rand,
+                      u, sp_points, loss_scale, lr_step_on_device=lr_step_on_device)
+    if world > 1:
+        allreduce_gradients(state.gbuf)   # pmean(grad) and pmean(stats) in one bucket
     # weight_l2 = sum(theta^2)/numel  ->  d/dtheta = 2*theta/numel  (train.py:101-108,114)
     wd = 2.0 * weight_decay_mult / model.params.numel() if weight_decay_mult else 0.0
     check(lib.pob_adam_update(model.sh_deg, model.num_mlps, ptr(model.params), ptr(state.grads), ptr(state.m),
@@ -217,7 +178,7 @@ def train_step(model, state, batch, lr, sparsity_weight=1e-3, sparsity_length=0.
 
 
 class GraphedTrainStep:
-    """One train_step captured in a CUDA graph (jitter draws, ~30 kernel launches, both gradient all-reduces, Adam,
+    """One train_step captured in a CUDA graph (jitter draws, ~30 kernel launches, the gradient all-reduce, Adam,
     operand re-pack) and replayed per step: at 512 rays per GPU (BASELINE's global batch of 4096 on 8 GPUs) the
     launches would otherwise cost as much as the kernels.  The batch lives in static device buffers; the learning
     rate and the step count reach the Adam kernel through a two-float device buffer written before every replay.

@@ -1,5 +1,5 @@
 """Per-layer-step cycle summary of CTA 0 of mlp_fwd (debug trace): epilogue, MMA phase, iteration period.
-usage: trace_summary.py <debug_flags> [save]   (env POB_PAIR=0/1 selects single-CTA / CTA-pair kernels)"""
+usage: trace_summary.py [save]   (save: with the training-mode stores)"""
 import os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -12,8 +12,7 @@ m = 148 * 256 * 6
 pts = (torch.rand((m, 3), device="cuda") * 3 - 1.5).contiguous()
 sig = torch.empty(m, device="cuda")
 tr = torch.zeros((5, 256), dtype=torch.int64, device="cuda")
-flags = int(sys.argv[1]) if len(sys.argv) > 1 else 0
-saving = len(sys.argv) > 2 and sys.argv[2] == "save"
+saving = len(sys.argv) > 1 and sys.argv[1] == "save"
 tiles = (m + 511) // 512 * 4
 sh = torch.empty(tiles * 8 * 65536, dtype=torch.uint8, device="cuda") if saving else None
 se = torch.empty(tiles * 16384, dtype=torch.uint8, device="cuda") if saving else None
@@ -22,7 +21,7 @@ ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
 for i in range(3):
     tr.zero_()
     if i == 2: ev[0].record()
-    check(lib.pob_debug_trace_fwd(ptr(blob), 3, ptr(pts), m, ptr(sig), ptr(tr), flags, ptr(sh), ptr(se), ptr(sm), None))
+    check(lib.pob_debug_trace_fwd(ptr(blob), 3, ptr(pts), m, ptr(sig), ptr(tr), ptr(sh), ptr(se), ptr(sm), None))
 ev[1].record()
 torch.cuda.synchronize()
 t = tr.cpu().numpy()
@@ -35,5 +34,5 @@ epi = (ee[:, 2] - ee[:, 0])[1:17]
 sigt = (ee[:, 3] - ee[:, 2])[1:17]
 ph = np.array([mm[k + k // 8][1] - mm[k + k // 8][0] for k in range(1, 17)])
 per = [int(mm[9 * (k + 1)][0] - mm[9 * k][0]) for k in range((len(mm) - 1) // 9)]
-print(f"PAIR={os.environ.get('POB_PAIR','1')} flags={flags} save={saving}: kernel {ev[0].elapsed_time(ev[1])*1e3:.0f} us | "
+print(f"save={saving}: kernel {ev[0].elapsed_time(ev[1])*1e3:.0f} us | "
       f"epilogue {epi.mean():.0f} signal {sigt.mean():.0f} MMA-phase {ph.mean():.0f} (min {ph.min()} max {ph.max()}) | iteration {np.mean(per):.0f} cycles")
